@@ -524,6 +524,31 @@ def file_to_tsdf(args, device, rank, world, grp):
     return res
 
 
+# ----------------------------------------------------------------------------- output dump
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(d, vol):
+    """Writes what the last timed step left in the volume, i.e. its last scene (the step resets the volume before each scene):
+    the volume's counters, every allocated block's coordinates (sorted), and sdf / weight / colour of the voxels of a fixed
+    seeded sample of those blocks (all of them when they fit), float32 / float64 .npy files of at most DUMP_BYTES in all."""
+    os.makedirs(d, exist_ok=True)
+    st = vol.stats()
+    xyz, vox = vol.download_blocks()
+    n = len(xyz)
+    per_block = 512 * 5 * 4 + 8                                  # sdf, weight, r, g, b as float32 + the block's index
+    k = min(n, (DUMP_BYTES - 12 * n - (1 << 16)) // per_block)
+    pick = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False)) if k < n else np.arange(n)
+    v = vox[pick]
+    out = {"stats": np.array([st.frames_integrated, st.frames_skipped, st.blocks_allocated, st.voxels_updated, st.blocks_visited], np.float64),
+           "block_xyz": xyz.astype(np.float32), "sample_block_index": pick.astype(np.float64),
+           "sample_sdf": v["sdf"].astype(np.float32), "sample_weight": v["w"].astype(np.float32),
+           "sample_rgb": np.stack([v["r"], v["g"], v["b"]], -1).astype(np.float32)}
+    for name, a in out.items():
+        np.save(os.path.join(d, name + ".npy"), a)
+    return {"dir": d, "blocks": n, "sampled_blocks": int(k), "bytes": int(sum(a.nbytes for a in out.values()))}
+
+
 # ----------------------------------------------------------------------------- GPU arm
 def load_traffic():
     try:
@@ -552,6 +577,7 @@ def main():
     ap.add_argument("--column-kernel", action="store_true", help="force the register-resident column kernel (SCN_TSDF_KERNEL_COLUMN)")
     ap.add_argument("--c3-frames", type=int, default=5578, help="frames of the configs[2] stand-in scan in the pipeline side section (0 = skip)")
     ap.add_argument("--parity-frames", type=int, default=64, help="frames of the in-bench parity check against the oracle (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the volume the last timed step computed to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -637,6 +663,7 @@ def main():
     frames_all, ms_dev = timed(step_dev)
     vol.sync()
     alloc_ms, integ_ms, n_batches, _ = vol.kernel_times()
+    dumped = dump_outputs(args.dump_outputs, vol) if args.dump_outputs and rank == 0 else None
     vol.close()
 
     # ---- pass 2: end to end from pinned host memory -------------------------------------------
@@ -723,6 +750,7 @@ def main():
                                  "the ncu capture) ~10x lower than that figure, so frac can exceed 1: the kernel is bound by instruction issue "
                                  "(issue_active), not by HBM; the two kernels of consecutive batches overlap, so their times sum to more than the step"},
             "parity_check": parity,
+            "dumped_outputs": dumped,
             "file_to_tsdf": f2t,
             "clocks": clocks,
         }

@@ -54,5 +54,31 @@ def main():
     print("wrote", os.path.join(G, "segmentator_golden.npz"))
 
 
+def fixtures(ref_root):
+    """Data files of the reference tree the tests read: the two ScanNet reconstruction parameter files, and the first
+    1000 vertices of the OBJ copy of gates381 with the faces among them (the whole file is 890 kB)."""
+    for name in ("zParametersScanNet.txt", "zParametersBundlingScanNet.txt"):
+        shutil.copyfile(os.path.join(ref_root, "Server", "tools", "recons", name), os.path.join(G, name))
+        os.chmod(os.path.join(G, name), 0o644)
+    keep, nv, lines = 1000, 0, []
+    with open(os.path.join(ref_root, "external", "mLib", "test", "testD3D11", "scans", "gates381.obj")) as fh:
+        for ln in fh:
+            if ln.startswith("v "):
+                nv += 1
+                if nv > keep:
+                    continue
+            elif ln.startswith("vn "):
+                if nv >= keep:
+                    continue
+            elif ln.startswith("f ") and max(int(x.split("/")[0]) for x in ln.split()[1:]) > keep:
+                continue
+            lines.append(ln)
+    with open(os.path.join(G, "gates381_head1000.obj"), "w") as fh:
+        fh.writelines(lines)
+
+
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:2] == ["fixtures"]:               # python scripts/make_golden.py fixtures <reference tree>
+        fixtures(sys.argv[2])
+    else:
+        main()

@@ -77,15 +77,17 @@ def test_obj_loader_semantics(tmp_path, built):
 
 
 def test_obj_matches_reference_on_gates381(tmp_path, built):
-    ref_so = os.path.join(os.path.dirname(G), "..", "oracle", "_ref", "libref_segmentator.so")
-    src = "/root/reference/external/mLib/test/testD3D11/scans/gates381.obj"
-    if not (os.path.exists(ref_so) and os.path.exists(src)):
-        pytest.skip("needs /root/reference")
+    """the first 1000 vertices of the reference's gates381.obj (scripts/make_golden.py) with the faces among them"""
     import oracle_bindings as ob
+    import reference_golden as rg
+    src = os.path.join(G, "gates381_head1000.obj")
     xyz, tri = mesh_load(src)
-    ref_ids = ob.ref_segment_file(src, len(xyz))
+    assert xyz.shape == (1000, 3) and len(tri) > 1000
+    with open(src, "rb") as fh:
+        inputs = rg.digest(fh.read())
+    ref_ids = rg.expect("gates381_head1000_obj", "libref_segmentator.so", inputs, lambda: rg.digest(ob.ref_segment_file(src, len(xyz))))
     ours = ob.oracle_segment(xyz, tri)          # same arrays -> same ids only if the loader parsed every float like tinyobj
-    assert (ours == ref_ids).all()
+    assert rg.digest(ours) == ref_ids
 
 
 def test_segs_json_bytes(tmp_path, built):

@@ -1,8 +1,8 @@
 """Pins the CPU oracles (test infrastructure) before anything is compared against them.
 
 * oracle/seg_oracle.c  vs  committed golden vectors produced by the UNMODIFIED reference
-  (tests/golden/segmentator_golden.npz, scripts/make_golden.py) and, where oracle/_ref exists, the reference
-  itself (libref_segmentator.so built from /root/reference by oracle/Makefile).
+  (tests/golden/segmentator_golden.npz, scripts/make_golden.py, and tests/golden/reference_digests.json), which the
+  reference itself (libref_segmentator.so, built by oracle/Makefile where the reference tree is present) is checked against.
 * oracle/tsdf_oracle.c has nothing to be pinned against ("parity unpinned": the reference ships no TSDF
   source); it is checked for internal consistency and against the analytic geometry of the synthetic scene."""
 import hashlib
@@ -12,11 +12,11 @@ import numpy as np
 import pytest
 
 import oracle_bindings as ob
+import reference_golden as rg
 from scannet_b200 import synth
 from scannet_b200._lib import TsdfParams
 
 G = os.path.join(os.path.dirname(__file__), "golden")
-HAVE_REF = os.path.exists(os.path.join(ob.ROOT, "oracle", "_ref", "libref_segmentator.so"))
 
 
 def golden():
@@ -49,7 +49,6 @@ def test_seg_oracle_sort_and_kruskal_golden(built):
     assert e.tobytes() == g["graph_edges_sorted"].tobytes()          # libstdc++ std::sort tie order
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 @pytest.mark.parametrize("n,kind", [(1000, "ties"), (100000, "ties"), (65536, "organ"), (300000, "rand"), (17, "ties"), (16, "ties"), (200000, "few")])
 def test_seg_oracle_sort_vs_reference_stdsort(built, n, kind):
     rng = np.random.default_rng(n)
@@ -63,17 +62,22 @@ def test_seg_oracle_sort_vs_reference_stdsort(built, n, kind):
     else:
         e["w"] = np.concatenate([np.arange(n // 2), np.arange(n - n // 2)[::-1]]).astype(np.float32)
     e["a"] = np.arange(n); e["b"] = rng.integers(0, n, n)
-    e1 = e.copy(); e2 = e.copy()
-    ob.ref_segmentator().ref_segment_graph(n + 1, n, e1.ctypes.data, 0.5, None, None)
+    e2 = e.copy()
     ob.seg_oracle().oracle_seg_sort_edges(e2.ctypes.data, n)
-    assert e1.tobytes() == e2.tobytes()
+
+    def ref():
+        e1 = e.copy()
+        ob.ref_segmentator().ref_segment_graph(n + 1, n, e1.ctypes.data, 0.5, None, None)
+        return rg.digest(e1)
+
+    assert rg.digest(e2) == rg.expect(f"stdsort_{kind}_{n}", "libref_segmentator.so", rg.digest(e), ref)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 def test_seg_oracle_vs_reference_feature_mesh(built, tmp_path):
     x, t = synth.make_feature_mesh(120, 90, seed=4)
     p = tmp_path / "f.ply"; synth.write_ply(p, x, t)
-    assert (ob.oracle_segment(x, t) == ob.ref_segment_file(p, len(x))).all()
+    ref = rg.expect("feature_mesh_120x90_s4", "libref_segmentator.so", rg.digest(x, t), lambda: rg.digest(ob.ref_segment_file(p, len(x))))
+    assert rg.digest(ob.oracle_segment(x, t)) == ref
 
 
 def test_tsdf_oracle_geometry(built):

@@ -1,13 +1,12 @@
 """CPU: the `key = value;` parameter files the reconstruction stage is launched with (Server/scan_processor.py:27-35) parse into
-scn_tsdf_params.  When the reference tree is present the REAL files are read where they lie; a committed excerpt of the same
-lines keeps the test meaningful on machines without it."""
+scn_tsdf_params: the reference's own files (copies in tests/golden/), and an excerpt of the same lines."""
 import os
 
 import pytest
 
 from scannet_b200 import tsdf
 
-REF = "/root/reference/Server/tools/recons"
+G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 EXCERPT = """\
 // excerpt of Server/tools/recons/zParametersScanNet.txt (lines 20-21, 34-35, 47-58) in the reference's own syntax
 s_sensorIdx = 8;	//0 kinect, 8 SensorDataReader
@@ -39,12 +38,11 @@ def test_excerpt_of_the_scannet_parameter_file(tmp_path, built):
     check_scannet(tsdf.params_from_file(str(f)))
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "zParametersScanNet.txt")), reason="reference tree not present")
 def test_real_reference_parameter_files(built):
-    p = tsdf.params_from_file(os.path.join(REF, "zParametersScanNet.txt"))
+    p = tsdf.params_from_file(os.path.join(G, "zParametersScanNet.txt"))
     check_scannet(p)
     # the bundling file switches the depth bilateral pre-filter on (zParametersBundlingScanNet.txt:72-74); files are applied in order
-    q = tsdf.params_from_file(os.path.join(REF, "zParametersBundlingScanNet.txt"), p)
+    q = tsdf.params_from_file(os.path.join(G, "zParametersBundlingScanNet.txt"), p)
     assert q.depth_filter == 1 and abs(q.depth_sigma_d - 2.0) < 1e-7 and abs(q.depth_sigma_r - 0.05) < 1e-7
     check_scannet(q)
 

@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 import oracle_bindings as ob
+import reference_golden as rg
 from scannet_b200 import synth, tsdf
 
 pytestmark = pytest.mark.gpu
@@ -44,29 +45,28 @@ def test_empty_volume_mesh(built):
     assert len(x) == 0 and len(t) == 0
 
 
+def segmentator_cli_digest(tool, d):
+    """stdout and segs.json bytes of `tool` on a copy of gates381.ply in directory d (default and explicit parameters), then
+    the usage text and status without arguments"""
+    d.mkdir()
+    shutil.copy(os.path.join(G, "gates381.ply"), d / "gates381.ply")
+    parts = []
+    for args, out in (((), "gates381.0.010000.segs.json"), (("0.05", "5"), "gates381.0.050000.segs.json")):
+        o = subprocess.run([tool, str(d / "gates381.ply"), *args], capture_output=True, text=True)
+        assert o.returncode == 0, o.stderr
+        parts += [o.stdout.replace(str(d), "X"), (d / out).read_bytes().replace(str(d).encode(), b"X")]
+    u = subprocess.run([tool], capture_output=True, text=True)
+    assert u.returncode == 255
+    return rg.digest(*parts, u.stdout)
+
+
 def test_segmentator_cli_matches_reference_binary(built, tmp_path):
     """same stdout, same <base>.0.010000.segs.json bytes as the unmodified reference binary"""
-    ref = os.path.join(ROOT, "oracle", "_ref", "segmentator_ref")
-    if not os.path.exists(ref):
-        pytest.skip("oracle/_ref not built")
-    a = tmp_path / "a"; b = tmp_path / "b"; a.mkdir(); b.mkdir()
-    for d in (a, b):
-        shutil.copy(os.path.join(G, "gates381.ply"), d / "gates381.ply")
-    o1 = subprocess.run([os.path.join(BIN, "segmentator"), str(a / "gates381.ply")], capture_output=True, text=True)
-    o2 = subprocess.run([ref, str(b / "gates381.ply")], capture_output=True, text=True)
-    assert o1.returncode == 0 and o2.returncode == 0, (o1.stderr, o2.stderr)
-    assert o1.stdout.replace(str(a), "X") == o2.stdout.replace(str(b), "X")
-    f1 = (a / "gates381.0.010000.segs.json").read_bytes(); f2 = (b / "gates381.0.010000.segs.json").read_bytes()
-    assert f1.replace(str(a).encode(), b"X") == f2.replace(str(b).encode(), b"X")
-    # explicit parameters + usage
-    o3 = subprocess.run([os.path.join(BIN, "segmentator"), str(a / "gates381.ply"), "0.05", "5"], capture_output=True, text=True)
-    o4 = subprocess.run([ref, str(b / "gates381.ply"), "0.05", "5"], capture_output=True, text=True)
-    assert o3.stdout.replace(str(a), "X") == o4.stdout.replace(str(b), "X")
-    assert (a / "gates381.0.050000.segs.json").read_bytes().replace(str(a).encode(), b"X") == \
-        (b / "gates381.0.050000.segs.json").read_bytes().replace(str(b).encode(), b"X")
-    u1 = subprocess.run([os.path.join(BIN, "segmentator")], capture_output=True, text=True)
-    u2 = subprocess.run([ref], capture_output=True, text=True)
-    assert u1.stdout == u2.stdout and u1.returncode == u2.returncode == 255
+    with open(os.path.join(G, "gates381.ply"), "rb") as fh:
+        inputs = rg.digest(fh.read())
+    ref = rg.expect("segmentator_cli_gates381", "segmentator_ref", inputs,
+                    lambda: segmentator_cli_digest(os.path.join(ROOT, "oracle", "_ref", "segmentator_ref"), tmp_path / "b"))
+    assert segmentator_cli_digest(os.path.join(BIN, "segmentator"), tmp_path / "a") == ref
 
 
 def test_fuse_then_segment_end_to_end(built, tmp_path):

@@ -1,41 +1,43 @@
 """CPU: the segs.json consumer oracle (oracle/segs_oracle.c) pinned against the real mLib operators
-(oracle/_ref/libref_mlib.so, compiled from /root/reference/external/mLib/include where it lies), plus the segs.json reader
-(host code, no GPU needed)."""
+(oracle/_ref/libref_mlib.so, compiled from the reference's external/mLib/include where it lies; their outputs are stored in
+tests/golden/reference_digests.json), plus the segs.json reader (host code, no GPU needed)."""
 import json
-import os
 
 import numpy as np
 import pytest
 
 import oracle_bindings as ob
+import reference_golden as rg
 from scannet_b200 import segs, synth
 
-HAVE_REF = os.path.exists(os.path.join(ob.ROOT, "oracle/_ref/libref_mlib.so"))
+
+def float_digest(a):
+    """digest of the float32 bits, every NaN counted as the same value"""
+    a = np.ascontiguousarray(a, np.float32)
+    return rg.digest(np.where(np.isnan(a), np.float32(np.nan), a))
 
 
-def same_floats(a, b):
-    a = np.ascontiguousarray(a, np.float32); b = np.ascontiguousarray(b, np.float32)
-    return bool(((a.view(np.uint32) == b.view(np.uint32)) | (np.isnan(a) & np.isnan(b))).all())
-
-
-@pytest.mark.skipif(not HAVE_REF, reason="compiled mLib shim not present (built where /root/reference exists)")
 def test_area_matches_mlib(built):
     rng = np.random.default_rng(3)
     tris = rng.normal(size=(4000, 3, 3)).astype(np.float32)
     tris[:50, 2] = tris[:50, 0] + 2 * (tris[:50, 1] - tris[:50, 0])            # collinear -> the 1e-5 cosine guard
     tris[50:60, 1] = tris[50:60, 0]                                            # zero-length side -> NaN cosine
-    o = ob.segs_oracle(); r = ob.ref_mlib()
+    o = ob.segs_oracle()
     a = np.array([o.oracle_tri_area_mlib(t[0].ctypes.data, t[1].ctypes.data, t[2].ctypes.data) for t in tris], np.float32)
-    b = np.array([r.ref_tri_area(t[0].ctypes.data, t[1].ctypes.data, t[2].ctypes.data) for t in tris], np.float32)
-    assert same_floats(a, b)
+
+    def ref():
+        r = ob.ref_mlib()
+        return float_digest(np.array([r.ref_tri_area(t[0].ctypes.data, t[1].ctypes.data, t[2].ctypes.data) for t in tris], np.float32))
+
+    assert float_digest(a) == rg.expect("mlib_triangle_area", "libref_mlib.so", rg.digest(tris), ref)
     assert (a[:50] == 0).all() and np.isnan(a[50:60]).all()
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="compiled mLib shim not present")
 @pytest.mark.parametrize("mesh", ["grid", "adversarial"])
 def test_vertex_normals_match_mlib(built, mesh):
     xyz, tri = synth.make_feature_mesh(60, 50, 1) if mesh == "grid" else synth.make_adversarial_mesh(0)
-    assert same_floats(ob.oracle_vertex_normals_mlib(xyz, tri), ob.ref_vertex_normals_mlib(xyz, tri))
+    ref = rg.expect(f"mlib_vertex_normals_{mesh}", "libref_mlib.so", rg.digest(xyz, tri), lambda: float_digest(ob.ref_vertex_normals_mlib(xyz, tri)))
+    assert float_digest(ob.oracle_vertex_normals_mlib(xyz, tri)) == ref
 
 
 def test_aggregate_oracle_matches_python_dicts(built):
