@@ -327,7 +327,7 @@ typedef struct scn_fuse_report {
   uint64_t device_bytes_in_use;    /* cudaMemGetInfo after fusion: volume + decode staging */
   double   fuse_s;                 /* first frame in -> last frame integrated, decode included */
   double   decode_wait_s;          /* of which the integrator waited for the decoders */
-  double   depth_decode_s, color_decode_s;   /* busy time of the two decoder threads (overlaps fuse_s) */
+  double   depth_decode_s, color_decode_s;   /* busy time of the two decoder threads (overlaps fuse_s); host decode: its one thread in depth_decode_s */
   double   integrate_s;            /* integrator: submit + wait for the GPU, all chunks */
   double   depth_pack_s, depth_kernel_s;     /* of depth_decode_s: host packing + upload issue, inflate kernel (CUDA events) */
   double   color_host_s, color_entropy_s, color_convert_s;   /* of color_decode_s: host parse + pack, Huffman+IDCT kernel, colour kernel */

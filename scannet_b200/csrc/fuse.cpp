@@ -6,16 +6,16 @@
 // the file: camera tracking / bundle adjustment is not part of this path), extracts the surface with marching cubes and
 // writes `<base>_vh.ply` in the VCGLIB layout the `segment` stage reads (Server/config/scan_stages.json:33-37).
 //
-// Decode.  Default ("gpu"): the COMPRESSED payloads are uploaded and decoded in HBM — depth by the inflate kernel
-// (csrc/inflate.cu), JPEG colour by the device JPEG decoder (csrc/jpeg_gpu.cu), which samples only the colour pixels the
-// depth image needs — in chunks of a few hundred frames, two decoder threads (depth, colour) one chunk ahead of the
-// integration, so no raw frame crosses PCIe or touches a host core.  "host" (SCN_FUSE_DECODE=host; automatic for PNG / raw
-// colour): a host thread pool inflates / decodes one chunk ahead and the frames are handed over in pinned memory.
+// Decode.  Both modes run one chunk pipeline: the frames with a valid pose are planned in chunks, and decode lanes fill
+// double-buffered frame arrays one chunk ahead of the integrator.  "gpu" (default for zlib or raw depth): the COMPRESSED payloads
+// are decoded in HBM — depth by the inflate kernel (csrc/inflate.cu), JPEG colour by csrc/jpeg_gpu.cu, which samples only the
+// colour pixels the depth image needs; raw depth is uploaded as it is, raw / PNG colour decoded by a host thread pool.  "host"
+// (SCN_FUSE_DECODE=host): a host thread pool decodes depth and colour into pinned memory; the GPU decoders are tested against it.
+#include <algorithm>
 #include <atomic>
 #include <chrono>
 #include <condition_variable>
 #include <functional>
-#include <memory>
 #include <mutex>
 #include <cmath>
 #include <cstdio>
@@ -55,8 +55,6 @@ class Pool {
   const std::function<void()>* fn_ = nullptr; unsigned pending_ = 0; unsigned long gen_ = 0; bool stop_ = false;
 };
 
-struct Chunk { uint16_t* depth = nullptr; uint8_t* rgb = nullptr; std::vector<float> poses; uint32_t n = 0; int rc = 0; std::string err; };
-
 double now_s() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
 // colour pixel for every depth pixel: K_c * K_d^-1 * (x, y, 1), nearest (sensorData.h:1577-1586 with identity extrinsics)
@@ -72,31 +70,26 @@ void build_color_lut(const scn_sens_info_t& in, std::vector<int32_t>& lut) {
   }
 }
 
-void decode_chunk(const scn_sens* s, const scn_sens_info_t& in, const std::vector<int32_t>& lut, bool use_color, uint64_t f0, uint32_t n, Chunk& c, Pool& pool) {
-  const size_t px = (size_t)in.depth_width * in.depth_height;
-  c.n = n; c.rc = 0; c.poses.assign((size_t)n * 16, 0.f);
-  std::atomic<uint32_t> next{0}; std::atomic<int> rc{0};
-  std::mutex err_m;
-  auto work = [&]() {
+// a decoded colour frame registered to the depth image: out[p] = col[lut[p]], black where lut[p] < 0
+void register_color(const std::vector<int32_t>& lut, const uint8_t* col, uint8_t* out) {
+  for (size_t p = 0; p < lut.size(); ++p) {
+    const int32_t q = lut[p];
+    if (q >= 0) { out[3 * p] = col[3 * (size_t)q]; out[3 * p + 1] = col[3 * (size_t)q + 1]; out[3 * p + 2] = col[3 * (size_t)q + 2]; }
+    else out[3 * p] = out[3 * p + 1] = out[3 * p + 2] = 0;
+  }
+}
+
+// decode(i, colour scratch of scratch_bytes) for the frames i < n of a chunk, on every thread of `pool`.  Stops at the first failure
+// and returns its code; its text, thread-local to the worker that failed, is set again on the calling thread.
+int decode_on_pool(Pool& pool, uint32_t n, size_t scratch_bytes, const std::function<int(uint32_t, uint8_t*)>& decode) {
+  std::atomic<uint32_t> next{0}; std::atomic<int> rc{0}; std::mutex err_m; std::string err;
+  pool.run([&]() {
     static thread_local std::vector<uint8_t> col;                               // kept per pool thread: no 1-4 MB allocation per chunk
-    col.resize(use_color ? (size_t)in.color_width * in.color_height * 3 : 0);
-    for (;;) {
-      const uint32_t i = next.fetch_add(1);
-      if (i >= n || rc.load()) break;
-      scn_sens_frame_meta(s, f0 + i, &c.poses[(size_t)i * 16], nullptr, nullptr, nullptr, nullptr);
-      if (c.poses[(size_t)i * 16] == -INFINITY) continue;                        // skipped by the integrator anyway
-      int r = scn_sens_frame_depth_u16(s, f0 + i, c.depth + (size_t)i * px);
-      if (!r && use_color) {
-        r = scn_sens_frame_color_rgb8(s, f0 + i, col.data());
-        if (!r) { uint8_t* o = c.rgb + (size_t)i * px * 3;
-          for (size_t p = 0; p < px; ++p) { const int32_t q = lut[p]; if (q >= 0) { o[3 * p] = col[3 * q]; o[3 * p + 1] = col[3 * q + 1]; o[3 * p + 2] = col[3 * q + 2]; } else o[3 * p] = o[3 * p + 1] = o[3 * p + 2] = 0; } }
-      }
-      // the error text is thread-local: capture it on the worker that failed
-      if (r) { std::lock_guard<std::mutex> l(err_m); if (!rc.load()) { c.err = scn_last_error(); rc.store(r); } }
-    }
-  };
-  pool.run(work);
-  c.rc = rc.load();
+    col.resize(scratch_bytes);
+    for (uint32_t i; (i = next.fetch_add(1)) < n && !rc.load();)
+      if (const int r = decode(i, col.data())) { std::lock_guard<std::mutex> l(err_m); if (!rc.load()) { err = scn_last_error(); rc.store(r); } }
+  });
+  return rc.load() ? scn::fail(rc.load(), "%s", err.c_str()) : SCN_OK;
 }
 
 // ---- one scene on one GPU ------------------------------------------------------------------------------------------------------
@@ -130,18 +123,191 @@ struct FrameBufs {
 scn::StagePool<FrameBufs>& frame_pool() { static auto* p = new scn::StagePool<FrameBufs>(); return *p; }
 scn::StagePool<VolSlot>& vol_pool() { static auto* p = new scn::StagePool<VolSlot>(); return *p; }
 
+// Chunk c lists the frames of [c * chunk, (c + 1) * chunk) that have a valid pose: a frame without one is never decoded
+// (sensorData.h:382), so a corrupt payload there cannot fail the run.
+struct ChunkPlan {
+  std::vector<uint64_t> frames; std::vector<float> poses;
+  std::vector<const uint8_t*> src[2]; std::vector<uint64_t> len[2];        // compressed depth [0] and colour [1]: views into the stream
+};
+
+struct Scene {
+  scn_sens* s = nullptr; scn_sens_info_t in; int device = 0;
+  size_t px = 0; uint32_t chunk = 0;                       // depth pixels per frame, frames per chunk
+  std::vector<int32_t> lut;                                // colour pixel of every depth pixel; empty = fused without colour
+  std::vector<ChunkPlan> plan;
+  uint16_t* depth[2] = {nullptr, nullptr}; uint8_t* rgb[2] = {nullptr, nullptr};   // the double-buffered frame arrays
+};
+
+// returns the number of frames without a pose
+uint64_t plan_chunks(Scene& sc) {
+  sc.plan.assign((sc.in.n_frames + sc.chunk - 1) / sc.chunk, ChunkPlan());
+  uint64_t skipped = 0;
+  for (uint64_t f = 0; f < sc.in.n_frames; ++f) {
+    float T[16]; uint64_t cb = 0, db = 0; const uint8_t* cp = nullptr; const uint8_t* dp = nullptr;
+    scn_sens_frame_meta(sc.s, f, T, nullptr, nullptr, &cb, &db); scn_sens_frame_payload(sc.s, f, &cp, &dp);
+    if (T[0] == -INFINITY) { ++skipped; continue; }
+    ChunkPlan& pl = sc.plan[f / sc.chunk];
+    pl.frames.push_back(f); pl.poses.insert(pl.poses.end(), T, T + 16);
+    pl.src[0].push_back(dp); pl.len[0].push_back(db); pl.src[1].push_back(cp); pl.len[1].push_back(cb);
+  }
+  return skipped;
+}
+
+// a decode lane fills its part (depth, colour or both) of a chunk's frames into buffer `b`; its time is added to *busy_s
+struct Lane { std::function<int(const ChunkPlan& pl, int b)> fill; double* busy_s; };
+
+// The pipeline of both decode modes.  Every lane runs on a thread of its own and fills chunk c into buffer c & 1 once
+// c < consumed + 2; the integrator waits for every lane of chunk c, integrates it and waits for the GPU, after which buffer c & 1
+// may be filled again.  The first failure stops every lane; its code is returned with its text.
+int run_chunks(const Scene& sc, scn_tsdf* vol, const std::vector<Lane>& lanes, decltype(&scn_tsdf_integrate_device) integrate, scn_fuse_report_t& rep) {
+  std::mutex m; std::condition_variable cv;
+  std::vector<uint64_t> filled(lanes.size(), 0);                                // chunks each lane has finished
+  uint64_t consumed = 0;                                                          // chunks whose buffers are free again
+  int rc = SCN_OK; std::string err;                                               // the first failure
+  auto failed = [&](int r) { { std::lock_guard<std::mutex> l(m); if (!rc) { rc = r; err = scn_last_error(); } } cv.notify_all(); };
+  std::vector<std::thread> th;
+  for (size_t k = 0; k < lanes.size(); ++k)
+    th.emplace_back([&, k]() {
+      scn_set_device(sc.device);
+      for (uint64_t c = 0; c < sc.plan.size(); ++c) {
+        { std::unique_lock<std::mutex> l(m); cv.wait(l, [&]() { return rc || c < consumed + 2; }); if (rc) return; }
+        const double t = now_s();
+        const int r = sc.plan[c].frames.empty() ? SCN_OK : lanes[k].fill(sc.plan[c], (int)(c & 1));
+        *lanes[k].busy_s += now_s() - t;
+        if (r) { failed(r); return; }
+        { std::lock_guard<std::mutex> l(m); filled[k] = c + 1; } cv.notify_all();
+      }
+    });
+  for (uint64_t c = 0; c < sc.plan.size(); ++c) {
+    const double tw0 = now_s();
+    { std::unique_lock<std::mutex> l(m); cv.wait(l, [&]() { return rc || *std::min_element(filled.begin(), filled.end()) > c; }); if (rc) break; }
+    rep.decode_wait_s += now_s() - tw0;
+    const ChunkPlan& pl = sc.plan[c];
+    if (!pl.frames.empty()) {
+      const double ti0 = now_s();
+      int r = integrate(vol, (uint32_t)pl.frames.size(), sc.depth[c & 1], sc.rgb[c & 1], pl.poses.data(), sc.in.depth_intrinsic);
+      if (!r) r = scn_tsdf_sync(vol);                                             // buffer c & 1 may be filled again now
+      if (r) { failed(r); break; }
+      rep.integrate_s += now_s() - ti0;
+    }
+    { std::lock_guard<std::mutex> l(m); consumed = c + 1; } cv.notify_all();
+  }
+  const double tt0 = now_s();
+  for (std::thread& t : th) t.join();
+  rep.teardown_s = now_s() - tt0;
+  return rc ? scn::fail(rc, "%s", err.c_str()) : SCN_OK;
+}
+
+// GPU decode: the frame arrays live in HBM; a depth lane (inflate kernel, or one upload per raw frame) and a colour lane (device
+// JPEG decoder, or for raw / PNG colour the host pool into a pinned chunk, registered to depth on the way, and one upload).  Host
+// decode: the frame arrays live in pinned memory, filled by one lane whose host pool decodes each frame's depth and registered
+// colour; scn_tsdf_integrate_batch uploads a chunk while the lane decodes the next one.
+int fuse_chunks(Scene& sc, bool gpu, unsigned threads, scn_tsdf* vol, scn_fuse_report_t& rep) {
+  const double t0 = now_s();
+  const size_t CH = sc.chunk, px = sc.px, col_bytes = (size_t)sc.in.color_width * sc.in.color_height * 3;
+  const bool use_color = !sc.lut.empty(), jpeg = sc.in.color_compression == 2;
+  scn::StagePool<FrameBufs>::Lease fb(frame_pool());
+  auto alloc = [&](int i, size_t bytes) { return gpu ? fb->take(i, bytes) : scn_host_alloc(bytes); };
+  int32_t* d_lut = nullptr; void* st_d = nullptr; void* st_c = nullptr; uint8_t* h_rgb = nullptr; int rc = SCN_OK;
+  for (int b = 0; b < 2 && !rc; ++b) {
+    sc.depth[b] = (uint16_t*)alloc(b, CH * px * 2);
+    if (use_color) sc.rgb[b] = (uint8_t*)alloc(2 + b, CH * px * 3);
+    if (!sc.depth[b] || (use_color && !sc.rgb[b])) rc = SCN_ERR_CUDA;
+  }
+  if (!rc && gpu && use_color && jpeg) rc = (d_lut = (int32_t*)scn_device_alloc(px * 4)) ? scn_memcpy_h2d(d_lut, sc.lut.data(), px * 4, nullptr) : SCN_ERR_CUDA;
+  if (!rc && gpu) rc = scn_stream_create(&st_d);
+  if (!rc && gpu) rc = scn_stream_create(&st_c);
+  rep.buffers_s = now_s() - t0;
+  // the host decoders: of every frame in host mode, of raw / PNG colour in GPU mode
+  Pool pool(!gpu ? threads - 1 : use_color && !jpeg ? std::max(1u, std::min(32u, std::thread::hardware_concurrency())) - 1 : 0);
+  std::vector<Lane> lanes;
+  if (!gpu) lanes.push_back({[&](const ChunkPlan& pl, int b) {                     // its time counts as depth decode
+    return decode_on_pool(pool, (uint32_t)pl.frames.size(), use_color ? col_bytes : 0, [&](uint32_t i, uint8_t* col) {
+      int q = scn_sens_frame_depth_u16(sc.s, pl.frames[i], sc.depth[b] + (size_t)i * px);
+      if (!q && use_color && !(q = scn_sens_frame_color_rgb8(sc.s, pl.frames[i], col))) register_color(sc.lut, col, sc.rgb[b] + (size_t)i * px * 3);
+      return q;
+    });
+  }, &rep.depth_decode_s});
+  if (gpu) lanes.push_back({[&](const ChunkPlan& pl, int b) {
+    const uint32_t n = (uint32_t)pl.frames.size();
+    if (sc.in.depth_compression == 1) {
+      const int r = scn_inflate_batch_device(pl.src[0].data(), pl.len[0].data(), n, (uint64_t)px * 2, sc.depth[b], st_d);
+      double ps = 0, km = 0; scn_inflate_last_timings(&ps, &km, nullptr, nullptr);
+      rep.depth_pack_s += ps; rep.depth_kernel_s += km * 1e-3;
+      return r;
+    }
+    for (uint32_t i = 0; i < n; ++i)                                               // raw depth: uploaded as it is
+      if (const int r = pl.len[0][i] < px * 2 ? scn::fail(SCN_ERR_FORMAT, "frame %llu: invalid data", (unsigned long long)pl.frames[i])
+                                              : scn_memcpy_h2d(sc.depth[b] + (size_t)i * px, pl.src[0][i], px * 2, st_d)) return r;
+    return SCN_OK;
+  }, &rep.depth_decode_s});
+  if (gpu && use_color && jpeg) lanes.push_back({[&](const ChunkPlan& pl, int b) {
+    uint32_t k = 0; double hs = 0, em = 0, cm = 0;
+    const int r = scn_jpeg_decode_batch_device(pl.src[1].data(), pl.len[1].data(), (uint32_t)pl.frames.size(), sc.in.color_width, sc.in.color_height,
+                                               d_lut, (uint32_t)px, sc.rgb[b], st_c, &k);
+    scn_jpeg_last_timings(&hs, &em, &cm);
+    rep.color_frames_on_device += k; rep.color_host_s += hs; rep.color_entropy_s += em * 1e-3; rep.color_convert_s += cm * 1e-3;
+    return r;
+  }, &rep.color_decode_s});
+  if (gpu && use_color && !jpeg) lanes.push_back({[&](const ChunkPlan& pl, int b) {
+    const uint32_t n = (uint32_t)pl.frames.size();
+    if (!h_rgb && !(h_rgb = (uint8_t*)scn_host_alloc(CH * px * 3))) return SCN_ERR_CUDA;
+    const int r = decode_on_pool(pool, n, col_bytes, [&](uint32_t i, uint8_t* col) {
+      const int q = scn_sens_frame_color_rgb8(sc.s, pl.frames[i], col);
+      if (!q) register_color(sc.lut, col, h_rgb + (size_t)i * px * 3);
+      return q;
+    });
+    return r ? r : scn_memcpy_h2d(sc.rgb[b], h_rgb, (size_t)n * px * 3, st_c);
+  }, &rep.color_decode_s});
+  if (!rc) rc = run_chunks(sc, vol, lanes, gpu ? scn_tsdf_integrate_device : scn_tsdf_integrate_batch, rep);
+  const double tt0 = now_s();
+  scn_device_free(d_lut); scn_stream_destroy(st_d); scn_stream_destroy(st_c); scn_host_free(h_rgb);
+  if (!gpu) for (int b = 0; b < 2; ++b) { scn_host_free(sc.depth[b]); scn_host_free(sc.rgb[b]); }
+  rep.teardown_s += now_s() - tt0;
+  return rc;
+}
+
+// counters, marching cubes and the PLY
+int finish(const SceneJob& job, scn_tsdf* vol, bool use_color, scn_fuse_report_t& rep) {
+  scn_tsdf_stats_t st;
+  if (const int rc = scn_tsdf_stats(vol, &st)) return rc;
+  rep.frames_integrated = st.frames_integrated; rep.frames_skipped = st.frames_skipped + rep.frames_skipped_pose;
+  rep.blocks_allocated = st.blocks_allocated; rep.voxels_updated = st.voxels_updated;
+  if (job.verbose)
+    printf("integrated %llu frames (%llu skipped: invalid pose) in %.3f s = %.1f frames/s incl. decode; %llu blocks, %llu voxel updates\n",
+           (unsigned long long)rep.frames_integrated, (unsigned long long)rep.frames_skipped, rep.fuse_s, rep.frames_integrated / std::max(rep.fuse_s, 1e-9),
+           (unsigned long long)st.blocks_allocated, (unsigned long long)st.voxels_updated);
+  size_t used = 0, total = 0; if (!scn_device_mem_info(&used, &total)) rep.device_bytes_in_use = used;
+  if (job.out_path.empty()) return SCN_OK;
+  const double tm0 = now_s();
+  float* xyz = nullptr; uint8_t* rgb = nullptr; uint32_t* tri = nullptr; uint64_t nV = 0, nF = 0;
+  int rc = scn_tsdf_extract_mesh(vol, &xyz, &rgb, &tri, &nV, &nF);
+  rep.mc_s = now_s() - tm0;
+  if (!rc) rc = scn_mesh_save_ply(job.out_path.c_str(), xyz, use_color ? rgb : nullptr, nV, tri, nF);
+  rep.ply_s = now_s() - tm0 - rep.mc_s;
+  rep.mesh_vertices = nV; rep.mesh_faces = nF;
+  if (!rc && job.verbose) printf("mesh written to %s with %llu vertices, %llu faces\n", job.out_path.c_str(), (unsigned long long)nV, (unsigned long long)nF);
+  scn_free(xyz); scn_free(rgb); scn_free(tri);
+  return rc;
+}
+
+// every failure of a scene reaches the caller with its own code, the .sens path in front of its text
+int scene_error(const SceneJob& job, int rc) { return scn::fail(rc, "%s: %s", job.sens_path.c_str(), scn_last_error()); }
+
+// setup -> plan -> run the chunks -> finish
 int fuse_scene(const SceneJob& job, scn_fuse_report_t* rep_out) {
   scn_fuse_report_t rep; memset(&rep, 0, sizeof(rep));
   rep.device = job.device;
   const double t_begin = now_s();
-  if (scn_set_device(job.device)) return SCN_ERR_CUDA;
-  std::thread warm([dev = job.device]() { scn_set_device(dev); scn_cuda_warmup(); });          // context creation overlaps reading the .sens file
-  scn_sens* s = nullptr;
-  const int open_rc = scn_sens_open(job.sens_path.c_str(), &s);
-  const std::string open_err = open_rc ? scn_last_error() : "";
-  warm.join();
-  if (open_rc) return scn::fail(open_rc, "%s", open_err.c_str());
-  scn_sens_info_t in; scn_sens_info(s, &in);
+  Scene sc; sc.device = job.device;
+  int rc = scn_set_device(job.device);
+  if (!rc) {
+    std::thread warm([dev = job.device]() { scn_set_device(dev); scn_cuda_warmup(); });          // context creation overlaps reading the .sens file
+    rc = scn_sens_open(job.sens_path.c_str(), &sc.s);
+    warm.join();
+  }
+  if (rc) return scene_error(job, rc);
+  const scn_sens_info_t& in = sc.in; scn_sens_info(sc.s, &sc.in);
   scn_tsdf_params p = job.params;
   p.width = in.depth_width; p.height = in.depth_height; p.depth_shift = in.depth_shift;   // integrate at the stream's depth resolution
   if (p.batch_frames == 0) p.batch_frames = 32;
@@ -149,201 +315,34 @@ int fuse_scene(const SceneJob& job, scn_fuse_report_t* rep_out) {
   if (job.verbose)
     printf("fusing %s: %llu frames %ux%u, voxel %.4f m, truncation %.3f+%.3f*d\n", job.sens_path.c_str(), (unsigned long long)in.n_frames, in.depth_width,
            in.depth_height, p.voxel_size, p.trunc_base, p.trunc_scale);
-  scn_tsdf* vol = nullptr;
   scn::StagePool<VolSlot>::Lease vs(vol_pool());
-  if (vs->vol && !memcmp(&vs->p, &p, sizeof(p))) {                                     // same volume layout as the previous scene on this GPU
-    vol = vs->vol;
-    if (scn_tsdf_reset(vol)) { const std::string e = scn_last_error(); vs->release(); scn_sens_close(s); return scn::fail(SCN_ERR_CUDA, "%s", e.c_str()); }
-    rep.volume_reused = 1;
-  } else {
-    vs->release();
-    if (scn_tsdf_create(&p, job.device, &vol)) { const std::string e = scn_last_error(); scn_sens_close(s); return scn::fail(SCN_ERR_CUDA, "%s", e.c_str()); }
-    vs->vol = vol; vs->p = p;
-  }
-  const size_t px = (size_t)in.depth_width * in.depth_height;
-  std::vector<int32_t> lut; if (use_color) build_color_lut(in, lut);
-  // decode mode
-  const bool gpu_able = in.depth_compression == 0 || in.depth_compression == 1;
-  const bool gpu_decode = gpu_able && !(job.decode_mode && !strcmp(job.decode_mode, "host"));
-  if (job.verbose)
-    printf("decode: %s\n", !gpu_decode ? "host thread pool" : (use_color && in.color_compression != 2) ? "GPU inflate (depth), host thread pool (raw / PNG colour)"
-                                                                                      : "GPU inflate (depth) + GPU JPEG (colour), compressed payloads uploaded");
-  rep.gpu_decode = gpu_decode ? 1 : 0;
-  const double t0 = now_s();
-  rep.setup_s = t0 - t_begin;
-  int rc = 0; std::string err;
-  auto fail_here = [&](const char* what) { if (!rc) { rc = 1; err = what && *what ? what : scn_last_error(); } };
-  if (gpu_decode) {
-    const char* ce = getenv("SCN_FUSE_CHUNK");
-    const uint32_t CH = (uint32_t)std::max(16, std::min(4096, ce ? atoi(ce) : 1024));   // frames per decode chunk: enough streams in flight for the one-warp-per-frame decoders
-    const uint64_t n_chunks = (in.n_frames + CH - 1) / CH;
-    uint16_t* d_depth[2] = {nullptr, nullptr}; uint8_t* d_rgb[2] = {nullptr, nullptr}; int32_t* d_lut = nullptr;
-    void* st_d = nullptr; void* st_c = nullptr;
-    scn::StagePool<FrameBufs>::Lease fb(frame_pool());
-    for (int b = 0; b < 2; ++b) {
-      d_depth[b] = (uint16_t*)fb->take(b, (size_t)CH * px * 2);
-      if (use_color) d_rgb[b] = (uint8_t*)fb->take(2 + b, (size_t)CH * px * 3);
-      if (!d_depth[b] || (use_color && !d_rgb[b])) fail_here(nullptr);
-    }
-    if (use_color && !rc) { d_lut = (int32_t*)scn_device_alloc(px * 4); if (!d_lut || scn_memcpy_h2d(d_lut, lut.data(), px * 4, nullptr)) fail_here(nullptr); }
-    if (!rc && (scn_stream_create(&st_d) || scn_stream_create(&st_c))) fail_here(nullptr);
-    rep.buffers_s = now_s() - t0;
-    // per chunk: the frames with a valid pose, compacted (a frame without a pose is never decoded: sensorData.h:382)
-    struct ChunkPlan { std::vector<uint64_t> frames; std::vector<float> poses; };
-    std::mutex m; std::condition_variable cv;
-    std::vector<int> depth_done(n_chunks, 0), color_done(n_chunks, 0);            // 1 = ready, -1 = failed
-    std::vector<ChunkPlan> plan(n_chunks);
-    uint64_t consumed = 0;                                                          // chunks whose buffers are free again
-    std::string dec_err; bool stop = false;
-    for (uint64_t c = 0; c < n_chunks; ++c) {
-      const uint64_t f0 = c * CH, f1 = std::min<uint64_t>(in.n_frames, f0 + CH);
-      for (uint64_t f = f0; f < f1; ++f) {
-        float T[16]; scn_sens_frame_meta(s, f, T, nullptr, nullptr, nullptr, nullptr);
-        if (T[0] == -INFINITY) { ++rep.frames_skipped_pose; continue; }
-        plan[c].frames.push_back(f); plan[c].poses.insert(plan[c].poses.end(), T, T + 16);
-      }
-    }
-    std::unique_ptr<Pool> color_pool;
-    if (use_color && in.color_compression != 2) color_pool.reset(new Pool(std::max(1u, std::min(32u, std::thread::hardware_concurrency())) - 1));
-    uint8_t* h_rgb = nullptr;
-    auto decoder = [&](bool is_color) {
-      scn_set_device(job.device);
-      std::vector<const uint8_t*> src; std::vector<uint64_t> len;
-      for (uint64_t c = 0; c < n_chunks; ++c) {
-        { std::unique_lock<std::mutex> l(m); cv.wait(l, [&]() { return stop || c < consumed + 2; }); if (stop) return; }
-        const ChunkPlan& pl = plan[c];
-        const uint32_t n = (uint32_t)pl.frames.size();
-        int r = 0; std::string e;
-        if (n) {
-          src.resize(n); len.resize(n);
-          for (uint32_t i = 0; i < n; ++i) {
-            const uint8_t* cp = nullptr; const uint8_t* dp = nullptr; uint64_t cb = 0, db = 0;
-            scn_sens_frame_payload(s, pl.frames[i], &cp, &dp);
-            scn_sens_frame_meta(s, pl.frames[i], nullptr, nullptr, nullptr, &cb, &db);
-            src[i] = is_color ? cp : dp; len[i] = is_color ? cb : db;
-          }
-          const double td0 = now_s();
-          if (is_color && in.color_compression != 2) {
-            // raw / PNG colour: host pool into a pinned chunk (registered to depth on the way), one upload
-            if (!h_rgb) h_rgb = (uint8_t*)scn_host_alloc((size_t)CH * px * 3);
-            if (!h_rgb) r = SCN_ERR_CUDA;
-            std::atomic<uint32_t> nx{0}; std::atomic<int> prc{0}; std::mutex pem; std::string perr;
-            auto work = [&]() {
-              static thread_local std::vector<uint8_t> col;
-              col.resize((size_t)in.color_width * in.color_height * 3);
-              for (;;) {
-                const uint32_t i = nx.fetch_add(1);
-                if (i >= n || prc.load() || r) break;
-                const int q = scn_sens_frame_color_rgb8(s, pl.frames[i], col.data());
-                if (q) { std::lock_guard<std::mutex> l(pem); if (!prc.load()) { perr = scn_last_error(); prc.store(q); } break; }
-                uint8_t* o = h_rgb + (size_t)i * px * 3;
-                for (size_t pp = 0; pp < px; ++pp) { const int32_t qq = lut[pp]; if (qq >= 0) { o[3 * pp] = col[3 * (size_t)qq]; o[3 * pp + 1] = col[3 * (size_t)qq + 1]; o[3 * pp + 2] = col[3 * (size_t)qq + 2]; } else o[3 * pp] = o[3 * pp + 1] = o[3 * pp + 2] = 0; }
-              }
-            };
-            if (!r) { color_pool->run(work); r = prc.load(); if (r) scn::fail(r, "%s", perr.c_str()); }
-            if (!r) r = scn_memcpy_h2d(d_rgb[c & 1], h_rgb, (size_t)n * px * 3, st_c);
-            if (!r) { std::lock_guard<std::mutex> l(m); rep.color_decode_s += now_s() - td0; }
-          } else if (is_color) {
-            uint32_t k = 0;
-            r = scn_jpeg_decode_batch_device(src.data(), len.data(), n, in.color_width, in.color_height, d_lut, (uint32_t)px, d_rgb[c & 1], st_c, &k);
-            double hs = 0, em = 0, cm = 0; scn_jpeg_last_timings(&hs, &em, &cm);
-            if (!r) { std::lock_guard<std::mutex> l(m); rep.color_frames_on_device += k; rep.color_decode_s += now_s() - td0;
-                      rep.color_host_s += hs; rep.color_entropy_s += em * 1e-3; rep.color_convert_s += cm * 1e-3; }
-          } else if (in.depth_compression == 1) {
-            r = scn_inflate_batch_device(src.data(), len.data(), n, (uint64_t)px * 2, d_depth[c & 1], st_d);
-            double ps = 0, km = 0; scn_inflate_last_timings(&ps, &km, nullptr, nullptr);
-            if (!r) { std::lock_guard<std::mutex> l(m); rep.depth_decode_s += now_s() - td0; rep.depth_pack_s += ps; rep.depth_kernel_s += km * 1e-3; }
-          } else {
-            for (uint32_t i = 0; i < n && !r; ++i) {
-              if (len[i] < px * 2) { r = scn::fail(SCN_ERR_FORMAT, "frame %llu: invalid data", (unsigned long long)pl.frames[i]); break; }
-              r = scn_memcpy_h2d(d_depth[c & 1] + (size_t)i * px, src[i], px * 2, st_d);
-            }
-          }
-          if (r) e = scn_last_error();
-        }
-        { std::lock_guard<std::mutex> l(m); (is_color ? color_done : depth_done)[c] = r ? -1 : 1; if (r && dec_err.empty()) dec_err = e; }
-        cv.notify_all();
-        if (r) return;
-      }
-    };
-    std::thread th_d, th_c;
-    if (!rc) { th_d = std::thread(decoder, false); if (use_color) th_c = std::thread(decoder, true); }
-    for (uint64_t c = 0; c < n_chunks && !rc; ++c) {
-      const double tw0 = now_s();
-      {
-        std::unique_lock<std::mutex> l(m);
-        cv.wait(l, [&]() { return depth_done[c] != 0 && (!use_color || color_done[c] != 0); });
-        if (depth_done[c] < 0 || (use_color && color_done[c] < 0)) { fail_here(dec_err.c_str()); break; }
-      }
-      rep.decode_wait_s += now_s() - tw0;
-      const ChunkPlan& pl = plan[c];
-      if (!pl.frames.empty()) {
-        const double ti0 = now_s();
-        if (scn_tsdf_integrate_device(vol, (uint32_t)pl.frames.size(), d_depth[c & 1], use_color ? d_rgb[c & 1] : nullptr, pl.poses.data(), in.depth_intrinsic)) { fail_here(nullptr); break; }
-        if (scn_tsdf_sync(vol)) { fail_here(nullptr); break; }                          // the buffers of this chunk may be overwritten now
-        rep.integrate_s += now_s() - ti0;
-      }
-      { std::lock_guard<std::mutex> l(m); consumed = c + 1; }
-      cv.notify_all();
-    }
-    const double tt0 = now_s();
-    { std::lock_guard<std::mutex> l(m); stop = true; }
-    cv.notify_all();
-    if (th_d.joinable()) th_d.join();
-    if (th_c.joinable()) th_c.join();
-    scn_device_free(d_lut); scn_stream_destroy(st_d); scn_stream_destroy(st_c); scn_host_free(h_rgb);
-    rep.teardown_s = now_s() - tt0;
-  } else {
-    // host decode is the bottleneck of this mode (one frame = ~2 ms inflate + ~1-3 ms JPEG on one core): up to 64 cores,
-    // chunks of two frames per worker
-    const unsigned threads = std::max(1u, std::min(64u, std::thread::hardware_concurrency()));
-    const uint32_t CH = std::max(32u, 2 * threads);
-    Pool pool(threads - 1);
-    Chunk ch[2];
-    for (Chunk& c : ch) { c.depth = (uint16_t*)scn_host_alloc(CH * px * 2); c.rgb = use_color ? (uint8_t*)scn_host_alloc(CH * px * 3) : nullptr;
-      if (!c.depth || (use_color && !c.rgb)) fail_here(nullptr); }
-    uint64_t f = 0; int cur = 0;
-    if (!rc && in.n_frames) decode_chunk(s, in, lut, use_color, 0, (uint32_t)std::min<uint64_t>(CH, in.n_frames), ch[0], pool);
-    while (f < in.n_frames && !rc) {
-      Chunk& c = ch[cur];
-      if (c.rc) { fail_here(c.err.c_str()); break; }
-      // the GPU consumes chunk `cur` asynchronously while the host decodes the next one into the other buffer
-      if (scn_tsdf_integrate_batch(vol, c.n, c.depth, c.rgb, c.poses.data(), in.depth_intrinsic)) { fail_here(nullptr); break; }
-      f += c.n;
-      if (f < in.n_frames) decode_chunk(s, in, lut, use_color, f, (uint32_t)std::min<uint64_t>(CH, in.n_frames - f), ch[cur ^ 1], pool);
-      if (scn_tsdf_sync(vol)) { fail_here(nullptr); break; }      // chunk `cur` may be overwritten next round
-      cur ^= 1;
-    }
-    for (Chunk& c : ch) { scn_host_free(c.depth); scn_host_free(c.rgb); }
-  }
-  rep.fuse_s = now_s() - t0;
+  if (vs->vol && !memcmp(&vs->p, &p, sizeof(p))) { rep.volume_reused = 1; rc = scn_tsdf_reset(vs->vol); }   // same volume layout as the previous scene on this GPU
+  else { vs->release(); vs->p = p; rc = scn_tsdf_create(&p, job.device, &vs->vol); }
   if (!rc) {
-    scn_tsdf_stats_t st; scn_tsdf_stats(vol, &st);
-    rep.frames_integrated = st.frames_integrated; rep.frames_skipped = st.frames_skipped + rep.frames_skipped_pose;
-    rep.blocks_allocated = st.blocks_allocated; rep.voxels_updated = st.voxels_updated;
+    sc.px = (size_t)in.depth_width * in.depth_height;
+    if (use_color) build_color_lut(in, sc.lut);
+    const bool gpu_decode = (in.depth_compression == 0 || in.depth_compression == 1) && !(job.decode_mode && !strcmp(job.decode_mode, "host"));
     if (job.verbose)
-      printf("integrated %llu frames (%llu skipped: invalid pose) in %.3f s = %.1f frames/s incl. decode; %llu blocks, %llu voxel updates\n",
-             (unsigned long long)rep.frames_integrated, (unsigned long long)rep.frames_skipped, rep.fuse_s, rep.frames_integrated / std::max(rep.fuse_s, 1e-9),
-             (unsigned long long)st.blocks_allocated, (unsigned long long)st.voxels_updated);
-    size_t used = 0, total = 0;
-    if (!scn_device_mem_info(&used, &total)) rep.device_bytes_in_use = used;
-    if (!job.out_path.empty()) {
-      const double tm0 = now_s();
-      float* xyz = nullptr; uint8_t* rgb = nullptr; uint32_t* tri = nullptr; uint64_t nV = 0, nF = 0;
-      if (scn_tsdf_extract_mesh(vol, &xyz, &rgb, &tri, &nV, &nF)) fail_here(nullptr);
-      rep.mc_s = now_s() - tm0;
-      if (!rc && scn_mesh_save_ply(job.out_path.c_str(), xyz, use_color ? rgb : nullptr, nV, tri, nF)) fail_here(nullptr);
-      rep.ply_s = now_s() - tm0 - rep.mc_s;
-      rep.mesh_vertices = nV; rep.mesh_faces = nF;
-      if (!rc && job.verbose) printf("mesh written to %s with %llu vertices, %llu faces\n", job.out_path.c_str(), (unsigned long long)nV, (unsigned long long)nF);
-      scn_free(xyz); scn_free(rgb); scn_free(tri);
-    }
+      printf("decode: %s\n", !gpu_decode ? "host thread pool" : (use_color && in.color_compression != 2) ? "GPU inflate (depth), host thread pool (raw / PNG colour)"
+                                                                                        : "GPU inflate (depth) + GPU JPEG (colour), compressed payloads uploaded");
+    rep.gpu_decode = gpu_decode ? 1 : 0;
+    const double t0 = now_s();
+    rep.setup_s = t0 - t_begin;
+    // frames per chunk.  GPU: enough streams in flight for the one-warp-per-frame decoders.  Host: decode is the bottleneck of this
+    // mode (one frame = ~2 ms inflate + ~1-3 ms JPEG on one core): up to 64 cores, two frames per thread.
+    const char* ce = getenv("SCN_FUSE_CHUNK");
+    const unsigned threads = std::max(1u, std::min(64u, std::thread::hardware_concurrency()));
+    sc.chunk = gpu_decode ? (uint32_t)std::max(16, std::min(4096, ce ? atoi(ce) : 1024)) : std::max(32u, 2 * threads);
+    rep.frames_skipped_pose = plan_chunks(sc);
+    rc = fuse_chunks(sc, gpu_decode, threads, vs->vol, rep);
+    rep.fuse_s = now_s() - t0;
+    if (!rc) rc = finish(job, vs->vol, use_color, rep);
   }
   if (rc) vs->release();                                       // do not hand a volume of unknown state to the next scene
-  scn_sens_close(s);
+  scn_sens_close(sc.s);
   rep.total_s = now_s() - t_begin;
   if (rep_out) *rep_out = rep;
-  return rc ? scn::fail(SCN_ERR_FORMAT, "%s: %s", job.sens_path.c_str(), err.c_str()) : SCN_OK;
+  return rc ? scene_error(job, rc) : SCN_OK;
 }
 
 std::string default_out(const std::string& sens_path) { return sens_path.substr(0, sens_path.size() - 5) + "_vh.ply"; }

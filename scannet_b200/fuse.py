@@ -5,7 +5,8 @@ from __future__ import annotations
 
 import ctypes as C
 
-from ._lib import TsdfParams, check, lib
+from ._lib import check, lib
+from .tsdf import default_params
 
 
 class FuseReport(C.Structure):
@@ -24,27 +25,21 @@ class FuseReport(C.Structure):
         return d
 
 
-def _params(**over) -> TsdfParams:
-    p = TsdfParams()
-    lib().scn_tsdf_default_params(C.byref(p))
-    for k, v in over.items():
-        setattr(p, k, v)
-    return p
-
-
 def fuse_scene(sens_path: str, out_ply: str | None = None, device: int = 0, decode_mode: str | None = None, **param_over) -> dict:
+    params = default_params(**param_over)
     rep = FuseReport()
-    check(lib().scn_fuse_scene(str(sens_path).encode(), str(out_ply).encode() if out_ply else None, C.byref(_params(**param_over)), C.c_int(device),
+    check(lib().scn_fuse_scene(str(sens_path).encode(), str(out_ply).encode() if out_ply else None, C.byref(params), C.c_int(device),
                                decode_mode.encode() if decode_mode else None, C.byref(rep)))
     return rep.as_dict()
 
 
 def fuse_many(sens_paths, out_plys=None, devices=(0,), decode_mode: str | None = None, **param_over):
+    params = default_params(**param_over)
     n = len(sens_paths)
     sp = (C.c_char_p * n)(*[str(p).encode() for p in sens_paths])
     op = (C.c_char_p * n)(*[(str(p).encode() if p else None) for p in (out_plys or [None] * n)])
     dv = (C.c_int * len(devices))(*devices)
     reps = (FuseReport * n)()
-    check(lib().scn_fuse_many(sp, op, C.c_uint32(n), C.byref(_params(**param_over)), dv, C.c_uint32(len(devices)),
+    check(lib().scn_fuse_many(sp, op, C.c_uint32(n), C.byref(params), dv, C.c_uint32(len(devices)),
                               decode_mode.encode() if decode_mode else None, reps))
     return [r.as_dict() for r in reps]

@@ -62,3 +62,17 @@ def test_fuse_report_binding_matches_the_library_struct():
     from scannet_b200._lib import lib
     lib().scn_fuse_report_sizeof.restype = C.c_size_t
     assert lib().scn_fuse_report_sizeof() == C.sizeof(fuse.FuseReport)
+
+
+def test_fuse_rejects_a_misspelt_parameter_before_running(built, monkeypatch):
+    """a keyword that is no field of scn_tsdf_params raises instead of fusing with the default"""
+    import pytest
+    from scannet_b200 import fuse
+
+    def driver_must_not_run():
+        raise AssertionError("the fusion driver was called")
+    monkeypatch.setattr(fuse, "lib", driver_must_not_run)
+    with pytest.raises(AttributeError, match="max_block"):
+        fuse.fuse_scene("scene.sens", max_block=1 << 20)
+    with pytest.raises(AttributeError, match="max_block"):
+        fuse.fuse_many(["scene.sens"], max_block=1 << 20)
